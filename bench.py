@@ -294,7 +294,6 @@ def reference_arm(args):
     if rank != 0:
         return
     from oracle import fd_oracle as orc
-    orc.build()
     cores = usable_cores()
     scale = args.cpu_scale
     run, nnz, fcalls, desc = cpu_jacobian_runner(args.workload, args.fdtype, cores, scale)
@@ -401,6 +400,37 @@ def build_gpu_problem(pkg, workload, fdtype, dev, rank, world, max_batch, use_gr
         J = pkg.zeros_colmajor(n, n, dev)
         return dict(J=J, f=f, x=x, cache=cache, nnz=n * n, n=n, ctx=ctx, keep=(w, bs), col0=0, ncl=n)
     raise SystemExit(f"unknown workload {workload}")
+
+
+DUMP_ELEMENTS = 4 << 20          # at most this many float64 values written by --dump-outputs: 32 MiB
+DUMP_SEED = 20261017
+
+
+def j_values_flat(pkg, J):
+    """J's values as the caller holds them after a call, flat in storage order: nzval (CSC), the band storage (banded),
+    or the dense matrix column by column (zeros_colmajor)."""
+    if isinstance(J, pkg.SparseMatrixCSC):
+        return J.nzval
+    if isinstance(J, pkg.BandedMatrix):
+        return J.data
+    return J.t().reshape(-1)
+
+
+def output_dumper(out_dir, name, a):
+    """Returns a function that writes the flat device array `a`, as it is when called, to out_dir/<name>.npy in float64.
+    An array longer than DUMP_ELEMENTS is sampled at sorted positions drawn from DUMP_SEED and its length alone (drawn
+    here, not when the function runs), so runs with the same arguments write files that compare entry for entry."""
+    import torch
+    pos = None
+    if a.numel() > DUMP_ELEMENTS:
+        pos = np.unique(np.random.default_rng(DUMP_SEED).integers(0, a.numel(), size=DUMP_ELEMENTS))
+        pos = torch.from_numpy(pos).to(a.device)
+
+    def dump():
+        out = Path(out_dir)
+        out.mkdir(parents=True, exist_ok=True)
+        np.save(out / f"{name}.npy", (a if pos is None else a[pos]).to(torch.float64).cpu().numpy())
+    return dump
 
 
 def analytic_parity(pkg, workload, fdtype, prob, samples=4096):
@@ -529,10 +559,10 @@ def roofline_record(info, fdtype, scat_ms, scat_n, tsteps, traffic_key):
                     "nonzero) and may exceed 1; traffic = ncu dram bytes per launch from the named capture"}
 
 
-def measure(pkg, step, plan, steps, warmup, barrier, dist_max=None, spin_s=0.0):
+def measure(pkg, step, plan, steps, warmup, barrier, dist_max=None, spin_s=0.0, after_timed=None):
     """first call already done by the caller; warm-up (>= 3 steps, optionally at least spin_s seconds so the clock sampler
-    sees the load), K timed steps between CUDA events, then an eager pass with the library's own events around the
-    scatter launches."""
+    sees the load), K timed steps between CUDA events, after_timed() (sees the last timed step's results), then an eager
+    pass with the library's own events around the scatter launches."""
     import torch
     for _ in range(max(warmup, 3)):
         step()
@@ -554,6 +584,8 @@ def measure(pkg, step, plan, steps, warmup, barrier, dist_max=None, spin_s=0.0):
     if dist_max is not None:
         ms_total = dist_max(ms_total)
     c1 = plan.counters()
+    if after_timed is not None:
+        after_timed()
     tsteps = min(steps, 20)
     plan.enable_timing(True)
     plan.read_timing()
@@ -565,8 +597,9 @@ def measure(pkg, step, plan, steps, warmup, barrier, dist_max=None, spin_s=0.0):
     return dict(ms_total=ms_total, ms_step=ms_total / steps, c0=c0, c1=c1, scat_ms=scat_ms, scat_n=scat_n, tsteps=tsteps)
 
 
-def run_single(pkg, workload, fdtype, dev, args, steps, spin_s=0.0, strategy=0, sample_clocks=False):
-    """One workload on one GPU: build, measure, parity record.  Returns (record, prob, plan, nnz)."""
+def run_single(pkg, workload, fdtype, dev, args, steps, spin_s=0.0, strategy=0, sample_clocks=False, dump_dir=None):
+    """One workload on one GPU: build, measure, parity record; with dump_dir, J's values after the last timed step go
+    to dump_dir/J.npy (output_dumper).  Returns (record, prob, plan, nnz)."""
     import torch
     prob = build_gpu_problem(pkg, workload, fdtype, dev, 0, 1, args.max_batch, args.graph, strategy=strategy)
     J, f, x, cache = prob["J"], prob["f"], prob["x"], prob["cache"]
@@ -585,9 +618,12 @@ def run_single(pkg, workload, fdtype, dev, args, steps, spin_s=0.0, strategy=0, 
     plan = cache._last_plan
     # nvidia-smi samples every 100 ms: the sampler runs over warm-up (>= spin_s of the same step), the timed region and the
     # kernel-timing pass — all the same kernel sequence under load — and not over problem construction
+    after = output_dumper(dump_dir, "J", j_values_flat(pkg, J)) if dump_dir else None
     clocks = Clocks(dev.index if dev.index is not None else 0) if sample_clocks else None
-    m = measure(pkg, step, plan, steps, args.warmup, barrier, spin_s=spin_s)
-    clk = clocks.stop() if clocks else None
+    try:
+        m = measure(pkg, step, plan, steps, args.warmup, barrier, spin_s=spin_s, after_timed=after)
+    finally:
+        clk = clocks.stop() if clocks else None          # never leave the nvidia-smi sampler running
     info = plan.info()
     nnz = prob["nnz"] if prob["nnz"] is not None else info["n_entries"]
     f_points = m["c1"]["f_points"] - m["c0"]["f_points"]
@@ -632,7 +668,7 @@ def gpu_arm(args):
     if args.group > 1:
         return gpu_arm_group(args, pkg, dev)
     rec, prob, plan, nnz = run_single(pkg, workload, fdtype, dev, args, args.steps, spin_s=args.spin, strategy=args.strategy,
-                                      sample_clocks=True)
+                                      sample_clocks=True, dump_dir=args.dump_outputs)
     clk = rec.pop("clocks")
     J, f, x = prob["J"], prob["f"], prob["x"]
     info = plan.info()
@@ -666,7 +702,6 @@ def gpu_arm(args):
     cpu = None
     if not args.no_cpu and workload in ("c1", "c2", "c4"):
         from oracle import fd_oracle as orc
-        orc.build()
         scale = 1.0 if workload != "c4" else 0.2
         run, cnnz, cf, desc = cpu_jacobian_runner(workload, fdtype, 1, scale)
         med, reps = time_cpu(run, budget_s=14.0, max_reps=5)
@@ -853,8 +888,10 @@ def gpu_arm_multi(args, pkg, dev, rank, world):
     first_call_ms = (time.perf_counter() - t_first) * 1e3
     plan = cache._last_plan
     clocks = Clocks(dev.index) if rank == 0 else None
-    m = measure(pkg, step, plan, args.steps, args.warmup, barrier, dist_max=dist_max, spin_s=args.spin)
-    clk = clocks.stop() if clocks else None
+    try:
+        m = measure(pkg, step, plan, args.steps, args.warmup, barrier, dist_max=dist_max, spin_s=args.spin)
+    finally:
+        clk = clocks.stop() if clocks else None
     info = plan.info()
     nnz = prob["nnz"]
     ms_step = m["ms_step"]
@@ -914,7 +951,6 @@ def gpu_arm_multi(args, pkg, dev, rank, world):
     cpu = None
     if rank == 0 and not args.no_cpu and workload == "c4":
         from oracle import fd_oracle as orc
-        orc.build()
         run, cnnz, cf, desc = cpu_jacobian_runner("c4", fdtype, 1, 0.2)
         med, reps = time_cpu(run, budget_s=10.0, max_reps=3)
         cpu = {"value": cnnz / med, "unit": "nnz/s", "cores": 1, "kind": "port",
@@ -1023,7 +1059,12 @@ def main():
                     help="--gpus 1 default run: skip the c2-central / c3 / c4 / c5 sub-records")
     ap.add_argument("--cpu-scale", type=float, default=1.0, dest="cpu_scale",
                     help="--impl reference: problem-size fraction per step (1.0 = the full configuration)")
+    ap.add_argument("--dump-outputs", default=None, dest="dump_outputs", metavar="DIR",
+                    help="single-GPU run: after the timed steps write J's values from the last one to DIR/J.npy (float64; "
+                         "a fixed, seeded sample of at most 4 Mi entries) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     explicit = args.workload is not None or args.fdtype is not None
     if args.workload is None:
@@ -1037,6 +1078,8 @@ def main():
     if args.group > 1:
         args.workload, args.extras = "c4", False
         args.fdtype = args.fdtype or "forward"
+    if args.dump_outputs and (args.impl != "ours" or max(args.gpus, world) > 1 or args.group > 1):
+        ap.error("--dump-outputs applies to the single-GPU run of this implementation (--impl ours, --gpus 1)")
     if args.steps is None:
         args.steps = 5 if args.impl == "reference" else {"c1": 500, "c2": 200, "c3": 50, "c4": 30, "c5": 5}[args.workload]
     if args.impl == "reference":

@@ -3,6 +3,7 @@ include/fdjac_b200.h declares (and nothing is silently missing from the ctypes t
 with the oracle, and compute entry points FAIL LOUDLY without a device (no CPU fallback)."""
 import ctypes as C
 import re
+import shutil
 import subprocess
 from pathlib import Path
 
@@ -12,14 +13,18 @@ import pytest
 ROOT = Path(__file__).resolve().parent.parent
 
 
-@pytest.fixture(scope="module")
-def pkg():
-    import __graft_entry__ as ge
+def _build_module():
     import importlib.util
     spec = importlib.util.spec_from_file_location("_fdjac_build", ROOT / "finitediff.jl_b200" / "build.py")
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
-    mod.build()
+    return mod
+
+
+@pytest.fixture(scope="module")
+def pkg():
+    import __graft_entry__ as ge
+    _build_module().build()
     import _bootstrap
     return _bootstrap.load_package()
 
@@ -57,7 +62,9 @@ def test_synth_header_symbols(pkg):
 
 
 def test_sm100a_only(pkg):
-    out = subprocess.run(["cuobjdump", "--list-elf", str(pkg._lib.LIB_PATH)], capture_output=True, text=True).stdout
+    # the toolkit that built the library, found the way build.py finds nvcc (PATH need not contain the CUDA bin directory)
+    cuobjdump = shutil.which("cuobjdump") or str(Path(_build_module().nvcc_path()).with_name("cuobjdump"))
+    out = subprocess.run([cuobjdump, "--list-elf", str(pkg._lib.LIB_PATH)], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 

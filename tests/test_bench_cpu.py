@@ -42,3 +42,26 @@ def test_config_is_shared_by_both_arms():
         for fd in ("forward", "central"):
             a, b = bench.workload_config(w, fd), bench.workload_config(w, fd)
             assert a == b and set(a) == {"workload", "l2"}
+
+
+def test_output_dumper_writes_a_fixed_bounded_sample(tmp_path):
+    small = torch.arange(1000, dtype=torch.float64)
+    big = torch.arange(bench.DUMP_ELEMENTS + 12345, dtype=torch.float64) * 0.5
+    for d in ("a", "b"):
+        for name, a in (("small", small), ("big", big)):
+            bench.output_dumper(tmp_path / d, name, a)()
+    for name in ("small", "big"):
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype == np.float64 and np.array_equal(a, b)
+    assert np.array_equal(np.load(tmp_path / "a" / "small.npy"), small.numpy())
+    sample = np.load(tmp_path / "a" / "big.npy")
+    # entries of `big` at distinct positions in storage order, no more than the budget
+    assert 0 < sample.size <= bench.DUMP_ELEMENTS and (np.diff(sample) > 0).all()
+    assert np.isin(sample, big.numpy()).all()
+    assert (tmp_path / "a" / "big.npy").stat().st_size <= 64 << 20
+    # the values are read when the dumper runs (after the timed steps), not when it is made
+    later = small.clone()
+    dump = bench.output_dumper(tmp_path / "c", "later", later)
+    later.fill_(7.0)
+    dump()
+    assert (np.load(tmp_path / "c" / "later.npy") == 7.0).all()
