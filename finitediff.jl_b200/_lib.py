@@ -14,7 +14,7 @@ LIB_PATH = HERE / "libfdjac_b200.so"
 SYNTH_PATH = HERE / "libfdjac_synth.so"
 
 FDB_OK, FDB_ERR_INVALID, FDB_ERR_CUDA, FDB_ERR_CALLBACK, FDB_ERR_NOMEM, FDB_ERR_UNSUPPORTED, FDB_ERR_NO_DEVICE = range(7)
-FDB_FORWARD, FDB_CENTRAL, FDB_COMPLEX = 0, 1, 2
+FDB_FORWARD, FDB_CENTRAL, FDB_COMPLEX, FDB_HCENTRAL = 0, 1, 2, 3
 FDB_J_CSC_NZVAL, FDB_J_DENSE, FDB_J_BAND, FDB_J_SLOTS = 0, 1, 2, 3
 # FDB_STEP_DEFAULT: relstep / absstep keyword not given (any other value, 0 included, is used as passed)
 STEP_DEFAULT = float("nan")
@@ -100,6 +100,8 @@ ABI_SYMBOLS = {
     "fdb_check_coloring_csc": (_int, [_i64, _i64, _vp, _vp, _vp, C.POINTER(_i64)]),
     "fdb_jvp_plan_create": (_int, [_PP, _i64, _i64, C.POINTER(PlanOpts)]),
     "fdb_jvp": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f64, _f64, _f64, _vp]),
+    "fdb_hessian_plan_create": (_int, [_PP, _i64, C.POINTER(PlanOpts)]),
+    "fdb_hessian": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _f64, _f64, _vp]),
     "fdb_host_alloc": (_int, [_PP, C.c_size_t]),
     "fdb_host_free": (_int, [_vp]),
     "fdb_device_alloc": (_int, [_PP, C.c_size_t]),
@@ -120,6 +122,7 @@ SYNTH_SYMBOLS = {
     "fdbs_lap5": (_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp]),
     "fdbs_ellrows": (_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp]),
     "fdbs_rank1": (_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp]),
+    "fdbs_hess_poly": (_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp]),
     "fdbs_fail": (_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp]),
     "fdbs_fill_x": (_int, [_vp, _i64, C.c_uint64, _vp]),
     "fdbs_flush_l2": (_int, [_vp, _i64, _vp]),
@@ -144,6 +147,10 @@ class EllCtx(C.Structure):
 
 class Rank1Ctx(C.Structure):
     _fields_ = [("n", _i64), ("d_w", _vp), ("d_block_sums", _vp), ("max_batch", _i64), ("calls", _i64)]
+
+
+class HessPolyCtx(C.Structure):
+    _fields_ = [("n", _i64), ("d_w", _vp), ("calls", _i64)]
 
 
 class FdbError(RuntimeError):

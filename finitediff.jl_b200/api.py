@@ -10,7 +10,9 @@ and error behaviour follow src/jacobians.jl:
     finite_difference_jacobian_(J, f, x, fdtype="forward", returntype, f_in; relstep, absstep, colorvec, sparsity)
                                                                        (cache-less, :446-455)
     resize_(cache, i)                                                  (:655-661)
-    default_relstep / compute_epsilon                                  (epsilons.jl:26-29,50-53,134-144)
+    default_relstep / compute_epsilon                                  (epsilons.jl:26-29,50-53,74-77,134-144)
+    JVPCache / finite_difference_jvp_                                  (src/jvp.jl)
+    HessianCache / finite_difference_hessian_ / finite_difference_hessian   (src/hessians.jl:67-292)
 
 (`!` is not a Python identifier character: `finite_difference_jacobian!` is spelled with a trailing underscore.)
 Index arrays keep Julia's convention: Int64, 1-based.  PyTorch is used only for device memory and streams.
@@ -31,7 +33,8 @@ from . import _lib as L
 __all__ = [
     "SparseMatrixCSC", "BandedMatrix", "Tridiagonal", "BandedBlockBandedMatrix", "DenseColumnBlock", "NativeFn", "JacobianCache", "Plan",
     "finite_difference_jacobian_", "finite_difference_jacobian_b", "resize_", "default_relstep", "compute_epsilon",
-    "zeros_colmajor", "pinned_empty",
+    "zeros_colmajor", "pinned_empty", "JVPCache", "finite_difference_jvp_", "HessianCache",
+    "finite_difference_hessian_", "finite_difference_hessian",
 ]
 
 _DEFAULT = object()
@@ -49,14 +52,21 @@ def _fdtype_code(fdtype) -> int:
     return _FDTYPES[fdtype]
 
 
+def _step_fdtype_code(fdtype) -> int:
+    """_fdtype_code, plus the Hessian's 'hcentral' (a step-size type only: no Jacobian plan takes it)."""
+    if (isinstance(fdtype, str) and fdtype.lstrip(":") == "hcentral") or (isinstance(fdtype, int) and fdtype == L.FDB_HCENTRAL):
+        return L.FDB_HCENTRAL
+    return _fdtype_code(fdtype)
+
+
 def default_relstep(fdtype, T=torch.float64) -> float:
-    """src/epsilons.jl:134-144"""
-    return L.lib().fdb_default_relstep(_fdtype_code(fdtype))
+    """src/epsilons.jl:134-144 ("hcentral": eps(Float64)^(1/4) = 2^-13)"""
+    return L.lib().fdb_default_relstep(_step_fdtype_code(fdtype))
 
 
 def compute_epsilon(fdtype, x: float, relstep: float, absstep: float, dir: float = 1.0) -> float:
-    """src/epsilons.jl:26-29 (forward) / :50-53 (central)"""
-    return L.lib().fdb_compute_epsilon(_fdtype_code(fdtype), float(x), float(relstep), float(absstep), float(dir))
+    """src/epsilons.jl:26-29 (forward) / :50-53 (central) / :74-77 (hcentral)"""
+    return L.lib().fdb_compute_epsilon(_step_fdtype_code(fdtype), float(x), float(relstep), float(absstep), float(dir))
 
 
 # ------------------------------------------------------------------------------------------------ array helpers
@@ -965,3 +975,177 @@ def _shape_of(J):
             return (J.shape[0], 1)
         return tuple(J.shape)
     raise TypeError(f"unsupported J type {type(J)}")
+
+
+# ------------------------------------------------------------------------------------------------ Hessian (src/hessians.jl)
+class _PyScalarFn:
+    """Wraps a scalar Python f(x) -> number on CUDA tensors as an fdb_fn with m = 1.  `batched=True` callables receive
+    the (batch, n) points at once and return `batch` values; otherwise f is called once per point with a 1-D tensor."""
+
+    def __init__(self, f: Callable, n: int, device: torch.device, batched: bool):
+        self.f, self.n, self.device, self.batched = f, n, device, batched
+        self.exc: Optional[BaseException] = None
+        self.calls = 0
+        self.cfunc = L.FDB_FN(self._tramp)
+
+    def _tramp(self, _ctx, p_fx, p_x, batch, ldfx, ldx, stream):
+        try:
+            cur = torch.cuda.current_stream(self.device)
+            ctx = None
+            if (stream or 0) != cur.cuda_stream:
+                ctx = torch.cuda.stream(torch.cuda.ExternalStream(stream or 0, device=self.device))
+                ctx.__enter__()
+            try:
+                fx = torch.as_tensor(_DevArray(p_fx, (batch,), (ldfx * 8,)), device=self.device)
+                x2 = torch.as_tensor(_DevArray(p_x, (batch, self.n), (ldx * 8, 8)), device=self.device)
+                if self.batched:
+                    self.calls += int(batch)
+                    out = torch.as_tensor(self.f(x2), dtype=torch.float64, device=self.device).reshape(-1)
+                    if out.numel() != batch:
+                        raise ValueError(f"batched f returned {out.numel()} values for {batch} points")
+                    fx.copy_(out)
+                else:
+                    for b in range(int(batch)):
+                        self.calls += 1
+                        fx[b] = self.f(x2[b])
+            finally:
+                if ctx is not None:
+                    ctx.__exit__(None, None, None)
+            return 0
+        except BaseException as e:  # never let an exception cross the C ABI
+            self.exc = e
+            return 1
+
+
+_NO_INPLACE = object()
+
+
+class HessianCache:
+    """Mirror of FiniteDiff.HessianCache{T, fdtype, inplace} (src/hessians.jl:1-6): fields xpp, xpm, xmp, xmm.
+
+        HessianCache(x, fdtype="hcentral", inplace=True)               allocating: four copies of x          (:83-89)
+        HessianCache(xpp, xpm, xmp, xmm, fdtype="hcentral", inplace)   non-allocating: aliases the arrays    (:67-73)
+
+    The four-array form without `inplace` throws, as the reference does: its default `_hessian_inplace(x)` (:69) names
+    a variable that does not exist there.  The B200 path builds its points in plan-owned memory and never writes the
+    cache arrays (their end state in the reference, x again, is dropped), so a cache built from another x of the same
+    length gives the same Hessian (finitedifftests.jl:608-614).  The immutable branch (inplace=False) computes the same
+    values.  Extra keywords (B200-specific): max_batch (points per callback; default: NativeFn.max_batch for a native f,
+    1024 for a Python f) and scratch_bytes (cap on the B copies of x)."""
+
+    def __init__(self, *args, fdtype=None, inplace=_NO_INPLACE, max_batch=None, scratch_bytes=0):
+        if len(args) >= 4 and all(isinstance(a, torch.Tensor) for a in args[:4]):
+            self.xpp, self.xpm, self.xmp, self.xmm = args[:4]
+            rest = list(args[4:])
+            if rest:
+                fdtype = rest.pop(0)
+            if rest:
+                inplace = rest.pop(0)
+            if inplace is _NO_INPLACE:
+                raise TypeError("HessianCache(xpp, xpm, xmp, xmm, fdtype) needs `inplace`: the reference's default "
+                                "_hessian_inplace(x) refers to an undefined `x` (hessians.jl:69)")
+            x = self.xpp
+        elif len(args) >= 1:
+            x = args[0]
+            rest = list(args[1:])
+            if rest:
+                fdtype = rest.pop(0)
+            if rest:
+                inplace = rest.pop(0)
+            if rest:
+                raise TypeError("HessianCache(x, fdtype, inplace) takes at most three positional arguments")
+            if not _is_cuda(x):
+                raise TypeError("HessianCache needs a CUDA float64 tensor (this path has no CPU implementation)")
+            self.xpp, self.xpm, self.xmp, self.xmm = x.clone(), x.clone(), x.clone(), x.clone()
+        else:
+            raise TypeError("HessianCache(x[, fdtype, inplace]) or HessianCache(xpp, xpm, xmp, xmm, fdtype, inplace)")
+        if not _is_cuda(x):
+            raise TypeError("HessianCache needs CUDA float64 tensors (this path has no CPU implementation)")
+        fdtype = "hcentral" if fdtype is None else fdtype
+        self.fdtype = fdtype.lstrip(":") if isinstance(fdtype, str) else fdtype
+        _step_fdtype_code(self.fdtype)
+        self.inplace = True if inplace is _NO_INPLACE else bool(inplace)
+        self.max_batch = None if max_batch is None else int(max_batch)
+        self.scratch_bytes = int(scratch_bytes)
+        self._plan = None
+        self._plan_key = None
+
+    def plan(self, n: int, device, max_batch: int) -> Plan:
+        key = (n, str(device), max_batch)
+        if self._plan is None or self._plan_key != key:
+            h = C.c_void_p()
+            o = _opts(_step_fdtype_code(self.fdtype), _device_index(device), max_batch=max_batch,
+                      scratch_bytes=self.scratch_bytes)
+            L.check(L.lib().fdb_hessian_plan_create(C.byref(h), n, C.byref(o)))
+            self._plan, self._plan_key = Plan(h.value), key
+        return self._plan
+
+
+def _hessian_ld(H: torch.Tensor, n: int) -> int:
+    """Leading dimension of an (n, n) float64 CUDA view with one unit stride.  H is symmetric bit for bit, so a
+    row-major view is filled as the column-major matrix it is the transpose of."""
+    if not isinstance(H, torch.Tensor) or not H.is_cuda or H.dtype != torch.float64:
+        raise TypeError("H must be a float64 CUDA tensor")
+    if H.dim() != 2 or tuple(H.shape) != (n, n):
+        raise ValueError(f"size(H) = {tuple(H.shape)} != ({n}, {n})")
+    if n <= 1:
+        return max(n, 1)
+    if H.stride(0) == 1:
+        return int(H.stride(1))
+    if H.stride(1) == 1:
+        return int(H.stride(0))
+    raise ValueError("H needs one unit stride (a column- or row-major view)")
+
+
+def finite_difference_hessian_(H, f, x, cache=None, *, relstep=None, absstep=None, stream=None):
+    """finite_difference_hessian!(H, f, x, cache::HessianCache; relstep, absstep) (src/hessians.jl:202-292), or — when
+    `cache` is None or an fdtype string — the cache-less form (:181-189).
+
+    H: (n, n) float64 CUDA tensor with one unit stride; every entry is written.
+    f: scalar function of a 1-D float64 CUDA tensor (called once per point), a callable with f.batched = True taking
+       the (B, n) points and returning B values, or a NativeFn (an fdb_fn writing one scalar per point).
+    x: float64 CUDA tensor (any shape; flattened like Julia's vec).  Never modified.  Returns None."""
+    if isinstance(cache, str) or cache is None:
+        cache = HessianCache(x, "hcentral" if cache is None else cache)                   # :187
+    if not isinstance(cache, HessianCache):
+        raise TypeError("cache must be a HessianCache, an fdtype string, or None")
+    if cache.fdtype != "hcentral":
+        raise AssertionError("fdtype == Val(:hcentral)")                                  # :206
+    if not _is_cuda(x) or x.dtype != torch.float64:
+        raise TypeError("x must be a float64 CUDA tensor: the B200 path has no CPU implementation")
+    xv = x.reshape(-1)
+    if not xv.is_contiguous():
+        xv = xv.contiguous()
+    n = xv.numel()
+    if cache.xpp.numel() != n:
+        raise ValueError(f"length(cache.xpp) = {cache.xpp.numel()} != length(x) = {n}")
+    ldH = _hessian_ld(H, n)
+    if isinstance(f, NativeFn):
+        addr, ctx, pyfn = f.address, f.ctx_ptr, None
+        batch = cache.max_batch or f.max_batch
+    else:
+        pyfn = _PyScalarFn(f, n, x.device, bool(getattr(f, "batched", False)))
+        addr, ctx = L.fn_address(pyfn.cfunc), None
+        batch = cache.max_batch or 1024
+    plan = cache.plan(n, x.device, batch)
+    if stream is None:
+        stream = torch.cuda.current_stream(x.device).cuda_stream
+    with torch.cuda.device(x.device):
+        st = L.lib().fdb_hessian(plan.handle, addr, ctx, xv.data_ptr(), H.data_ptr(), ldH,
+                                 L.STEP_DEFAULT if relstep is None else float(relstep),
+                                 L.STEP_DEFAULT if absstep is None else float(absstep), C.c_void_p(stream))
+    if st == L.FDB_ERR_CALLBACK and pyfn is not None and pyfn.exc is not None:
+        exc, pyfn.exc = pyfn.exc, None
+        raise exc                                          # user f threw: propagate like Julia does
+    L.check(st)
+    cache._last_plan = plan
+    return None
+
+
+def finite_difference_hessian(f, x, cache=None, *, relstep=None, absstep=None, stream=None) -> torch.Tensor:
+    """finite_difference_hessian(f, x[, cache]; relstep, absstep) (src/hessians.jl:140-167): a new (n, n) float64
+    tensor, symmetric bit for bit (the reference wraps it in Symmetric)."""
+    n = x.numel()
+    H = torch.zeros((n, n), dtype=torch.float64, device=x.device)                        # mutable_zeromatrix(x) :164
+    finite_difference_hessian_(H, f, x, cache, relstep=relstep, absstep=absstep, stream=stream)
+    return H

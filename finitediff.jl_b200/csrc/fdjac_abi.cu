@@ -28,6 +28,7 @@
 #include "kernels_staged.cuh"
 #include "kernels_jvp.cuh"
 #include "kernels_color.cuh"
+#include "kernels_hessian.cuh"
 
 using namespace fdb;
 
@@ -57,7 +58,7 @@ static fdb_status fail(fdb_status st, const char *fmt, ...) {
     if (s__ != FDB_OK) return s__;   \
   } while (0)
 
-enum { SP_NONE = 0, SP_CSC = 1, SP_COO = 3, SP_BANDED = 4, SP_JVP = 5, SP_EPS = 6 };
+enum { SP_NONE = 0, SP_CSC = 1, SP_COO = 3, SP_BANDED = 4, SP_JVP = 5, SP_EPS = 6, SP_HESS = 7 };
 
 struct DeviceGuard {
   int prev = -1;
@@ -171,6 +172,9 @@ struct fdb_plan {
   // dense-column plans
   int64_t col_begin = 0, col_end = 0;
   double *eps_cols = nullptr;
+  // Hessian plans: the 2n^2+1 point values, F[p] at hess_F[p + 1] (so F[1] is 16-byte aligned, see hess_combine)
+  double *hess_F = nullptr;
+  int64_t hess_points = 0;
   // host-buffer path
   cudaStream_t hstream = nullptr;
   double *h_dx = nullptr, *h_dJ = nullptr, *h_dfx = nullptr, *h_dfin = nullptr;
@@ -736,9 +740,10 @@ int fdb_device_count(void) {
 double fdb_default_relstep(int fdtype) {
   if (fdtype == FDB_FORWARD) return sqrt(DBL_EPSILON);
   if (fdtype == FDB_CENTRAL) return cbrt(DBL_EPSILON);
+  if (fdtype == FDB_HCENTRAL) return 0x1p-13;   // eps(T)^(1/4) = (2^-52)^(1/4): exactly 2^-13
   return 1.0;
 }
-// src/epsilons.jl:26-29 / :50-53
+// src/epsilons.jl:26-29 / :50-53 / :74-77 (central and hcentral take no dir)
 double fdb_compute_epsilon(int fdtype, double x, double relstep, double absstep, double dir) {
   const double a = relstep * fabs(x);
   const double e = a > absstep ? a : absstep;
@@ -1092,11 +1097,13 @@ fdb_status fdb_plan_info(const fdb_plan *P, fdb_plan_info_t *info) {
   info->n_entries = P->E;
   info->j_len = P->j_len;
   info->n_colors = P->C;
-  const int64_t n_local = P->sp_kind == SP_NONE ? P->col_end - P->col_begin : (int64_t)P->local_colors.size();
+  const int64_t n_local = P->sp_kind == SP_NONE ? P->col_end - P->col_begin
+                          : P->sp_kind == SP_HESS ? P->n : (int64_t)P->local_colors.size();
   info->n_local_colors = n_local;
   info->n_groups = P->n_groups;
   info->slabs = P->slabs;
   info->fcalls_per_jacobian = P->fdtype == FDB_CENTRAL ? 2 * n_local : (P->fdtype == FDB_COMPLEX ? n_local : 1 + n_local);
+  if (P->sp_kind == SP_HESS) info->fcalls_per_jacobian = P->hess_points;   // 2n^2+1 (hessians.jl:209,233,269)
   info->device_bytes = (int64_t)P->device_bytes;
   info->fdtype = P->fdtype;
   info->jkind = P->jkind;
@@ -1155,7 +1162,7 @@ fdb_status fdb_plan_color_owner(const fdb_plan *P, int32_t *owner_out, int64_t c
 fdb_status fdb_plan_get_eps(fdb_plan *P, double *h_eps, int64_t cap, void *stream) {
   if (!P || !h_eps) return fail(FDB_ERR_INVALID, "NULL argument");
   DeviceGuard g(P->device);
-  const int64_t count = P->sp_kind == SP_NONE ? P->col_end - P->col_begin : P->C;   // JVP plans: C == 1
+  const int64_t count = P->sp_kind == SP_NONE ? P->col_end - P->col_begin : P->C;   // JVP plans: C == 1; Hessian plans: C == n
   if (cap < count) return fail(FDB_ERR_INVALID, "h_eps too small (%lld < %lld)", (long long)cap, (long long)count);
   const double *src = P->sp_kind == SP_NONE ? P->eps_cols : P->eps;
   if (count > 0) {
@@ -1193,7 +1200,7 @@ fdb_status fdb_plan_read_timing(fdb_plan *P, double *scatter_ms, int64_t *scatte
 fdb_status fdb_plan_set_peers(fdb_plan *P, int n_peers, double *const *peer_J) {
   if (!P) return fail(FDB_ERR_INVALID, "NULL plan");
   if (n_peers < 0 || n_peers > 64) return fail(FDB_ERR_INVALID, "n_peers out of range");
-  if (P->sp_kind == SP_NONE || P->sp_kind == SP_BANDED)
+  if (P->sp_kind == SP_NONE || P->sp_kind == SP_BANDED || P->sp_kind == SP_HESS)
     return fail(FDB_ERR_UNSUPPORTED, "peer stores are implemented for the entry-driven (CSC / COO) scatters");
   DeviceGuard g(P->device);
   if (!P->d_peers) TRY(P->alloc_t(&P->d_peers, 64));
@@ -1681,6 +1688,7 @@ fdb_status fdb_jacobian(fdb_plan *P, fdb_fn f, void *ctx, const double *d_x, dou
   if (!P || !f) return fail(FDB_ERR_INVALID, "NULL plan or f");
   if ((P->n > 0 && !d_x) || (P->j_len > 0 && !d_J)) return fail(FDB_ERR_INVALID, "NULL x or J");
   if (P->sp_kind == SP_JVP) return fail(FDB_ERR_INVALID, "this is a JVP plan: call fdb_jvp");
+  if (P->sp_kind == SP_HESS) return fail(FDB_ERR_INVALID, "this is a Hessian plan: call fdb_hessian");
   if (P->sp_kind == SP_EPS) return fail(FDB_ERR_INVALID, "this is a step-size plan: call fdb_color_eps");
   if (P->fdtype == FDB_COMPLEX && !P->complex_entry)
     return fail(FDB_ERR_INVALID, "this plan is a complex-step plan: call fdb_jacobian_complex with a complex128 callback");
@@ -1776,7 +1784,8 @@ fdb_status fdb_eps_plan_create(fdb_plan **plan, int64_t n, const int64_t *colorv
 fdb_status fdb_color_eps(fdb_plan *P, const double *d_x, double relstep, double absstep, double dir, double *d_eps_out,
                          void *stream) {
   if (!P) return fail(FDB_ERR_INVALID, "NULL plan");
-  if (P->sp_kind == SP_NONE || P->sp_kind == SP_JVP) return fail(FDB_ERR_INVALID, "fdb_color_eps needs a coloured plan");
+  if (P->sp_kind == SP_NONE || P->sp_kind == SP_JVP || P->sp_kind == SP_HESS)
+    return fail(FDB_ERR_INVALID, "fdb_color_eps needs a coloured plan");
   if (P->n > 0 && !d_x) return fail(FDB_ERR_INVALID, "NULL x");
   DeviceGuard g(P->device);
   if (!g.ok) return fail(FDB_ERR_CUDA, "cannot select device %d", P->device);
@@ -1792,7 +1801,7 @@ fdb_status fdb_color_eps(fdb_plan *P, const double *d_x, double relstep, double 
 
 fdb_status fdb_plan_set_external_eps(fdb_plan *P, const double *d_eps) {
   if (!P) return fail(FDB_ERR_INVALID, "NULL plan");
-  if (P->sp_kind == SP_NONE || P->sp_kind == SP_JVP || P->sp_kind == SP_EPS)
+  if (P->sp_kind == SP_NONE || P->sp_kind == SP_JVP || P->sp_kind == SP_EPS || P->sp_kind == SP_HESS)
     return fail(FDB_ERR_INVALID, "external step sizes apply to coloured Jacobian plans");
   P->ext_eps = d_eps;
   return FDB_OK;
@@ -1863,10 +1872,97 @@ fdb_status fdb_jvp(fdb_plan *P, fdb_fn f, void *ctx, double *d_jvp, const double
   return FDB_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ Hessian (src/hessians.jl:202-292)
+fdb_status fdb_hessian_plan_create(fdb_plan **plan, int64_t n, const fdb_plan_opts *opts) {
+  if (!plan) return fail(FDB_ERR_INVALID, "plan output pointer is NULL");
+  *plan = nullptr;
+  if (!opts || opts->fdtype != FDB_HCENTRAL)   // @assert fdtype == Val(:hcentral)   hessians.jl:206
+    return fail(FDB_ERR_UNSUPPORTED, "finite_difference_hessian supports only the hcentral fdtype (%d)", FDB_HCENTRAL);
+  if (opts->world > 1) return fail(FDB_ERR_UNSUPPORTED, "Hessian plans run on one GPU (world > 1 given)");
+  if (opts->use_graph) return fail(FDB_ERR_UNSUPPORTED, "Hessian plans do not capture CUDA graphs (use_graph = 1 given)");
+  if (n > ((int64_t)1 << 26))
+    return fail(FDB_ERR_NOMEM, "n = %lld: the 2n^2+1 point values would not fit in device memory", (long long)n);
+  // the Jacobian plans' common set-up validates forward / central / complex; the Hessian's own type is set afterwards
+  fdb_plan_opts o = *opts;
+  o.fdtype = FDB_CENTRAL;
+  fdb_plan *P = nullptr;
+  TRY(new_plan(plan, &o, 1, n));
+  P = *plan;
+  DeviceGuard g(P->device);
+  P->fdtype = FDB_HCENTRAL;
+  P->sp_kind = SP_HESS;
+  P->jkind = FDB_J_DENSE;
+  P->C = (int32_t)n;
+  P->ldF = 1;
+  P->ldx = std::max<int64_t>(2, (n + 1) & ~(int64_t)1);
+  P->hess_points = 2 * n * n + 1;
+  int64_t batch = opts->max_batch > 1 ? opts->max_batch : 1;
+  const int64_t budget = opts->scratch_bytes > 0 ? opts->scratch_bytes : (int64_t)8 << 30;
+  batch = std::max<int64_t>(1, std::min<int64_t>(batch, budget / (8 * P->ldx)));
+  batch = std::min<int64_t>(batch, P->hess_points);
+  P->batch = batch;
+  P->slabs = batch;
+  P->n_groups = (P->hess_points + batch - 1) / batch;
+  P->j_len = n * n;
+  P->E = n * n;
+  PLAN_TRY(P->alloc_t(&P->hess_F, (size_t)P->hess_points + 1));
+  PLAN_TRY(P->alloc_t(&P->xp, (size_t)batch * P->ldx));
+  PLAN_TRY(P->alloc_t(&P->eps, (size_t)std::max<int64_t>(n, 1)));
+  // combine pass: F read once, the n steps, H written once
+  P->alg_bytes = 8 * P->hess_points + 8 * n + 8 * n * n;
+  return FDB_OK;
+}
+
+fdb_status fdb_hessian(fdb_plan *P, fdb_fn f, void *ctx, const double *d_x, double *d_H, int64_t ldH, double relstep,
+                       double absstep, void *stream) {
+  if (!P || !f) return fail(FDB_ERR_INVALID, "NULL plan or f");
+  if (P->sp_kind != SP_HESS) return fail(FDB_ERR_INVALID, "not a Hessian plan (fdb_hessian_plan_create)");
+  const int64_t n = P->n;
+  if (n > 0 && (!d_x || !d_H)) return fail(FDB_ERR_INVALID, "NULL x or H");
+  if (ldH < n) return fail(FDB_ERR_INVALID, "ldH = %lld < n = %lld", (long long)ldH, (long long)n);
+  DeviceGuard g(P->device);
+  if (!g.ok) return fail(FDB_ERR_CUDA, "cannot select device %d", P->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  resolve_steps(FDB_HCENTRAL, relstep, absstep);                    // hessians.jl:204-205
+  double *F = P->hess_F + 1;                                        // F + 1 is 16-byte aligned (hess_combine)
+  if (n == 0) {                                                     // fx = f(x); the loops are empty     :209
+    TRY(call_f(P, f, ctx, F, P->xp, 1, s));
+    P->cnt.jacobians += 1;
+    return FDB_OK;
+  }
+  // e_k = compute_epsilon(Val(:hcentral) / Val(:central), x_k, relstep, absstep): one formula    :223, :234, :252
+  component_eps<<<(int)((n + kThreads - 1) / kThreads), kThreads, 0, s>>>(d_x, 0, n, 1, relstep, absstep, 1.0, P->eps);
+  hess_replicate<<<P->grid(n * P->batch), kThreads, 0, s>>>(d_x, n, P->ldx, P->batch, P->xp);
+  P->cnt.kernel_launches += 2;
+  const int64_t total = P->hess_points, B = P->batch;
+  int64_t prev_p0 = 0, prevB = 0;
+  for (int64_t p0 = 0; p0 < total; p0 += B) {
+    const int64_t kc = std::min<int64_t>(B, total - p0);
+    const int64_t slots = std::max(kc, prevB);
+    hess_points<<<(unsigned)((slots + kThreads - 1) / kThreads), kThreads, 0, s>>>(d_x, P->eps, n, p0, kc, prev_p0, prevB,
+                                                                                P->ldx, P->xp);
+    P->cnt.kernel_launches += 1;
+    TRY(call_f(P, f, ctx, F + p0, P->xp, kc, s));                  // f(x), f(_xpp), f(_xmm), f(_xpm), ...
+    prev_p0 = p0;
+    prevB = kc;
+  }
+  {
+    const int64_t nt = (n + kHessTile - 1) / kHessTile;
+    ScatterTimer tm(P, s);
+    hess_combine<<<dim3((unsigned)nt, (unsigned)nt), kThreads, 0, s>>>(F, P->eps, n, d_H, ldH);   // :233, :269, :291
+  }
+  P->cnt.kernel_launches += 1;
+  P->cnt.scatter_launches += 1;
+  CU(cudaGetLastError());
+  P->cnt.jacobians += 1;
+  return FDB_OK;
+}
+
 fdb_status fdb_jacobian_host(fdb_plan *P, fdb_fn f, void *ctx, const double *h_x, double *h_J, double *h_fx,
                              const double *h_f_in, double relstep, double absstep, double dir) {
   if (!P || !f) return fail(FDB_ERR_INVALID, "NULL plan or f");
   if ((P->n > 0 && !h_x) || (P->j_len > 0 && !h_J)) return fail(FDB_ERR_INVALID, "NULL x or J");
+  if (P->sp_kind == SP_HESS) return fail(FDB_ERR_INVALID, "this is a Hessian plan: call fdb_hessian");
   DeviceGuard g(P->device);
   if (!g.ok) return fail(FDB_ERR_CUDA, "cannot select device %d", P->device);
   if (!P->hstream) {

@@ -171,6 +171,31 @@ __global__ void __launch_bounds__(kT) k_tridiag_c(double2 *__restrict__ fx, cons
   }
 }
 
+// Scalar f(x) = sum w_i x_i^3 + sum x_i x_{i+1} + (sum x_i)^2/(2n), one warp per point.  Lane l sums the terms of
+// components l, l+32, ... in ascending order; xor butterfly; lane 0 forms (A + B) + (S*S)/(2n) — the order of
+// oracle_hessian/synth_scalar.c:synth_hess_poly.
+__global__ void __launch_bounds__(kT) k_hess_poly(double *__restrict__ fx, const double *__restrict__ x, int64_t n,
+                                                 const double *__restrict__ w, int64_t batch, int64_t ldfx, int64_t ldx) {
+  const int64_t p = blockIdx.x * (int64_t)(kT / 32) + (threadIdx.x >> 5);
+  if (p >= batch) return;
+  const int lane = threadIdx.x & 31;
+  const double *xb = x + p * ldx;
+  double a = 0.0, b = 0.0, s = 0.0;
+  for (int64_t i = lane; i < n; i += 32) {
+    const double xi = xb[i];
+    a = add(a, mul(__ldg(w + i), mul(mul(xi, xi), xi)));
+    if (i + 1 < n) b = add(b, mul(xi, xb[i + 1]));
+    s = add(s, xi);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    a = add(a, __shfl_xor_sync(0xffffffffu, a, o));
+    b = add(b, __shfl_xor_sync(0xffffffffu, b, o));
+    s = add(s, __shfl_xor_sync(0xffffffffu, s, o));
+  }
+  if (lane == 0) fx[p * ldfx] = add(add(a, b), __ddiv_rn(mul(s, s), (double)(2 * n)));
+}
+
 __device__ __forceinline__ uint64_t splitmix64_at(uint64_t seed, uint64_t i) {
   uint64_t z = seed + (i + 1) * 0x9E3779B97F4A7C15ULL;
   z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ULL;
@@ -273,6 +298,19 @@ int fdbs_rank1(void *vctx, double *d_fx, const double *d_x, int64_t batch, int64
   const int vec_ok = (((uintptr_t)d_x | (uintptr_t)d_fx | (uintptr_t)c->d_w) & 15) == 0 && (ldx & 1) == 0 && (ldfx & 1) == 0;
   dim3 g2((unsigned)blocks_for((c->n + 3) / 4, 128), (unsigned)batch);
   k_rank1<<<g2, kT, 0, (cudaStream_t)stream>>>(d_fx, d_x, c->n, c->d_w, c->d_block_sums, nblk, ldfx, ldx, vec_ok);
+  return cudaGetLastError() == cudaSuccess ? 0 : 3;
+}
+
+int fdbs_hess_poly(void *vctx, double *d_fx, const double *d_x, int64_t batch, int64_t ldfx, int64_t ldx, void *stream) {
+  fdbs_hess_poly_ctx *c = (fdbs_hess_poly_ctx *)vctx;
+  if (!c || batch < 1) return 1;
+  c->calls += batch;
+  if (c->n <= 0) {   // f of the empty vector: every sum is 0
+    if (cudaMemset2DAsync(d_fx, (size_t)ldfx * 8, 0, 8, (size_t)batch, (cudaStream_t)stream) != cudaSuccess) return 3;
+    return 0;
+  }
+  k_hess_poly<<<(unsigned)((batch + kT / 32 - 1) / (kT / 32)), kT, 0, (cudaStream_t)stream>>>(d_fx, d_x, c->n, c->d_w, batch,
+                                                                                            ldfx, ldx);
   return cudaGetLastError() == cudaSuccess ? 0 : 3;
 }
 

@@ -17,16 +17,19 @@
 #     DeviceTridiagonal J (structured, COO) src/iteration_utils.jl:25-32 with ArrayInterface.findstructralnz
 #     CuMatrix J + dense 0/1 prototype      src/jacobians.jl:473-488, 526-527
 #     CuMatrix J, sparsity === nothing      src/jacobians.jl:548-557, 590-598 (dense column branch, colorvec quirk included)
-#   for Val(:forward), Val(:central) and Val(:complex) (src/jacobians.jl:623-648), plus the JVP and the multi-GPU group.
-# Everything else of FiniteDiff.jl (CPU arrays, gradients, hessians, out-of-place forms) keeps using the stock package.
+#   for Val(:forward), Val(:central) and Val(:complex) (src/jacobians.jl:623-648), plus the JVP, the multi-GPU group and
+#   the Hessian of a scalar function (finite_difference_hessian!, src/hessians.jl:202-292: the stock cache-less and
+#   out-of-place forms reach it through HessianCache(x) / mutable_zeromatrix(x) on a CuVector).
+# Everything else of FiniteDiff.jl (CPU arrays, gradients, out-of-place Jacobians) keeps using the stock package.
 module FiniteDiffB200
 
 using FiniteDiff, SparseArrays, CUDA
-import FiniteDiff: finite_difference_jacobian!, finite_difference_jvp!, JacobianCache, JVPCache
+import FiniteDiff: finite_difference_jacobian!, finite_difference_jvp!, finite_difference_hessian!, JacobianCache, JVPCache,
+                  HessianCache
 
 const libfdjac = get(ENV, "FDJAC_B200_LIB", "libfdjac_b200.so")
 
-const FDB_FORWARD, FDB_CENTRAL, FDB_COMPLEX = Cint(0), Cint(1), Cint(2)
+const FDB_FORWARD, FDB_CENTRAL, FDB_COMPLEX, FDB_HCENTRAL = Cint(0), Cint(1), Cint(2), Cint(3)
 const FDB_J_CSC_NZVAL, FDB_J_DENSE, FDB_J_BAND, FDB_J_SLOTS = Cint(0), Cint(1), Cint(2), Cint(3)
 const FDB_STEP_DEFAULT = NaN            # relstep / absstep keyword not given (include/fdjac_b200.h)
 
@@ -410,6 +413,77 @@ function finite_difference_jvp!(jvp::CuVector{Float64}, f, x::CuVector{Float64},
                 CuPtr{Float64}, Float64, Float64, Float64, Ptr{Cvoid}),
             plan.handle, cf, pointer_from_objref(st), pointer(jvp), pointer(x), pointer(v), pointer(cache.x1), pointer(cache.fx1),
             f_in === nothing ? CU_NULL : pointer(f_in), stepval(relstep), stepval(absstep), Float64(dir), CUDA.stream().handle)
+    end
+    st.err === nothing || throw(st.err)
+    check(rc)
+    nothing
+end
+
+# ---- Hessian: finite_difference_hessian!(H, f, x, cache::HessianCache; relstep, absstep)   src/hessians.jl:202-292
+# f(x::CuVector) returns a number and is called once per point; wrap it in BatchedScalar(f, max_batch) when it can take
+# the points of a batch at once: f(X) with X an n x B CuMatrix view (column b = point b) returning B numbers.
+struct BatchedScalar{F}
+    f::F
+    max_batch::Int
+end
+
+const HESSIAN_PLANS = Dict{Tuple{Int, Int}, Plan}()
+
+function hessian_plan(n::Integer, max_batch::Integer)
+    lock(PLANS_LOCK) do
+        get!(HESSIAN_PLANS, (Int(n), Int(max_batch))) do
+            h = Ref{Ptr{Cvoid}}(C_NULL)
+            opts = Ref(PlanOpts(FDB_HCENTRAL; max_batch = max_batch))
+            check(ccall((:fdb_hessian_plan_create, libfdjac), Cint, (Ref{Ptr{Cvoid}}, Int64, Ref{PlanOpts}), h, n, opts))
+            Plan(h[])
+        end
+    end
+end
+
+# fdb_fn with m = 1: point b's scalar goes to fx[b*ldfx]
+function scalar_trampoline(ctx::Ptr{Cvoid}, fx::CuPtr{Float64}, x::CuPtr{Float64}, batch::Int64, ldfx::Int64, ldx::Int64,
+        stream::Ptr{Cvoid})::Cint
+    st = unsafe_pointer_to_objref(ctx)::FnState
+    try
+        if st.f isa BatchedScalar
+            X = view(unsafe_wrap(CuArray, x, (Int(ldx), Int(batch))), 1:st.n, :)
+            vals = st.f.f(X)
+            copyto!(unsafe_wrap(CuArray, fx, Int(batch)), Float64.(vals))       # ldfx == 1
+        else
+            for b in 0:(batch - 1)
+                xv = unsafe_wrap(CuArray, x + b * ldx * sizeof(Float64), st.n)
+                fill!(unsafe_wrap(CuArray, fx + b * ldfx * sizeof(Float64), 1), Float64(st.f(xv)))
+            end
+        end
+        return Cint(0)
+    catch err
+        st.err = err
+        return Cint(1)
+    end
+end
+
+"""
+    finite_difference_hessian!(H::CuMatrix{Float64}, f, x::CuVector{Float64}, cache::HessianCache; relstep, absstep)
+
+Same signature and keyword meaning as `src/hessians.jl:202-205`; `fdtype` must be `Val(:hcentral)` (`:206`).  The cache
+arrays are not used (the points are built in plan-owned memory) and keep their contents.  Every entry of `H` is
+written; `H[j,i]` is a bit copy of `H[i,j]` (`copytri!`, `:291`).
+"""
+function finite_difference_hessian!(H::CuMatrix{Float64}, f, x::CuVector{Float64},
+        cache::HessianCache{T, fdtype, inplace};
+        relstep = nothing, absstep = relstep) where {T, fdtype, inplace}
+    @assert fdtype == Val(:hcentral)
+    n = length(x)
+    size(H) == (n, n) || throw(DimensionMismatch("size(H) != (length(x), length(x))"))
+    plan = hessian_plan(n, f isa BatchedScalar ? f.max_batch : 1)
+    st = FnState(f, 1, n, nothing)
+    cf = @cfunction(scalar_trampoline, Cint, (Ptr{Cvoid}, CuPtr{Float64}, CuPtr{Float64}, Int64, Int64, Int64, Ptr{Cvoid}))
+    rc = Cint(0)
+    GC.@preserve st H x begin
+        rc = ccall((:fdb_hessian, libfdjac), Cint,
+            (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, CuPtr{Float64}, CuPtr{Float64}, Int64, Float64, Float64, Ptr{Cvoid}),
+            plan.handle, cf, pointer_from_objref(st), pointer(x), pointer(H), Int64(ld(H)), stepval(relstep),
+            stepval(absstep), CUDA.stream().handle)
     end
     st.err === nothing || throw(st.err)
     check(rc)

@@ -48,8 +48,10 @@ typedef enum {
 
 /* fdtype — the Val(:forward)/Val(:central)/Val(:complex) type parameter of JacobianCache (jacobians.jl:1-9).
  * FDB_COMPLEX is the complex-step colour loop (jacobians.jl:623-648): x + im*eps, J = imag(f)/eps, eps = eps(Float64);
- * plans of that type are driven through fdb_jacobian_complex with a complex128 callback. */
-enum { FDB_FORWARD = 0, FDB_CENTRAL = 1, FDB_COMPLEX = 2 };
+ * plans of that type are driven through fdb_jacobian_complex with a complex128 callback.
+ * FDB_HCENTRAL is the Val(:hcentral) parameter of HessianCache (hessians.jl:1-6): only Hessian plans take it
+ * (fdb_hessian_plan_create), and the Hessian plan takes nothing else (hessians.jl:206). */
+enum { FDB_FORWARD = 0, FDB_CENTRAL = 1, FDB_COMPLEX = 2, FDB_HCENTRAL = 3 };
 
 /* Where `J[row, col] = v` lands — what the reference decides by dispatch on typeof(J). */
 typedef enum {
@@ -140,7 +142,8 @@ const char *fdb_last_error(void);
 /* number of usable CUDA devices (0 => every compute entry point returns FDB_ERR_NO_DEVICE) */
 int fdb_device_count(void);
 
-/* ---- step size: src/epsilons.jl:134-144 / :26-29,50-53 (host-side scalars, for callers and tests) ---- */
+/* ---- step size: src/epsilons.jl:134-144 / :26-29,50-53,74-77 (host-side scalars, for callers and tests).
+ *      FDB_HCENTRAL: default relstep eps(Float64)^(1/4) = 2^-13; the step is max(relstep*|x|, absstep), no dir. ---- */
 double fdb_default_relstep(int fdtype);
 double fdb_compute_epsilon(int fdtype, double x, double relstep, double absstep, double dir);
 
@@ -313,6 +316,33 @@ fdb_status fdb_check_coloring_csc(int64_t m, int64_t n, const int64_t *colptr, c
 fdb_status fdb_jvp_plan_create(fdb_plan **plan, int64_t m, int64_t n, const fdb_plan_opts *opts);
 fdb_status fdb_jvp(fdb_plan *plan, fdb_fn f, void *ctx, double *d_jvp, const double *d_x, const double *d_v, double *d_x1,
                    double *d_fx1, const double *d_f_in, double relstep, double absstep, double dir, void *stream);
+
+/* ---- Hessian of a scalar function: finite_difference_hessian!(H, f, x, cache::HessianCache; relstep, absstep)
+ *      src/hessians.jl:202-292.  The reference makes 2n^2+1 scalar calls one at a time; here they are batched points:
+ *        p = 0                      f(x)
+ *        row i (0-based) at R(i) = 1 + 2i(2n-i):  x+e_i*E_i, x-e_i*E_i, then for j = i+1..n-1 the four points with
+ *                                   components (i, j) moved by (+,+), (+,-), (-,+), (-,-)       (:226-227, :239-260)
+ *      every other component is exactly x (the reference restores by assignment, :272-275, :284-289).  Step
+ *      e_k = max(relstep*|x_k|, absstep) for the diagonal and the off-diagonal alike (:223, :234, :252).
+ *        H[i,i] = ((F[R] - 2 F[0]) + F[R+1]) / (e_i*e_i)                                          (:233)
+ *        H[i,j] = (((F[q] - F[q+1]) - F[q+2]) + F[q+3]) / ((4 e_i)*e_j),  q = R(i)+2+4(j-i-1)      (:268-269)
+ *        H[j,i] = H[i,j] bit for bit                                                              (copytri!, :291)
+ *   fdb_hessian_plan_create: opts->fdtype must be FDB_HCENTRAL (anything else: FDB_ERR_UNSUPPORTED, as :206 asserts);
+ *      opts->max_batch = points per callback (0/1: one); opts->scratch_bytes caps the B copies of x (0: 8 GiB);
+ *      world > 1 and use_graph = 1 are FDB_ERR_UNSUPPORTED.  The plan owns the 2n^2+1 values F (16 n^2 bytes,
+ *      allocated here: FDB_ERR_NOMEM when that fails).
+ *   fdb_hessian: f is an fdb_fn with m = 1: point b's scalar goes to d_fx[b*ldfx] (ldfx = 1; d_fx is 8-byte aligned).
+ *      d_x: n doubles (device), never written.  d_H: dense column-major n x n, leading dimension ldH >= n (device);
+ *      every one of the n^2 entries is written, rows [n, ldH) of each column are not touched.  relstep / absstep:
+ *      FDB_STEP_DEFAULT as for fdb_jacobian.  Stream-ordered, no host synchronisation.
+ *   Other entry points: fdb_jacobian / fdb_jvp / fdb_color_eps / fdb_plan_set_external_eps reject a Hessian plan
+ *      (FDB_ERR_INVALID) and fdb_hessian rejects every other plan; fdb_plan_get_eps returns the n steps of the last call;
+ *      fdb_plan_info: m = 1, n_colors = n, fcalls_per_jacobian = 2n^2+1, moved_bytes_scatter = the combine kernel's
+ *      compulsory bytes (F read once, eps, H written once); fdb_plan_counters / fdb_plan_enable_timing count and time
+ *      the combine launch as the scatter launch. ---- */
+fdb_status fdb_hessian_plan_create(fdb_plan **plan, int64_t n, const fdb_plan_opts *opts);
+fdb_status fdb_hessian(fdb_plan *plan, fdb_fn f, void *ctx, const double *d_x, double *d_H, int64_t ldH, double relstep,
+                       double absstep, void *stream);
 
 /* ---- helpers for hosts without their own CUDA bindings ---- */
 fdb_status fdb_host_alloc(void **p, size_t bytes);  /* pinned host memory */
